@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mpixels/s of the projection-remap hot path on synthetic 8K equirect frames (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2|cfg3|cfg4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2|cfg3|cfg4] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one yuv420p frame (3 planes) through the hot path ([segmented low-pass] -> gather).  Default
@@ -205,10 +205,33 @@ class DeviceFrames:
         self.out_args = [[(t.data_ptr(), t.stride(0)) for t in fr] for fr in self.d_out]
 
 
-def measure_config(name, cfg, ctx, spec, K, warmup, dev, rank, world, barrier, want_e2e, e2e_steps):
+DUMP_LIMIT_BYTES = 64_000_000 - 4096  # --dump-outputs: at most 64 MB in all, .npy headers included
+
+
+def dump_outputs(dump_dir, spec, planes):
+    """Writes the output planes of one frame as float32 DIR/out_{y,u,v}.npy: whole planes while the frame fits
+    DUMP_LIMIT_BYTES as float32 (cfg2 does), else the same seeded sample of rows of every plane in every run."""
+    import numpy as np
+    import torch
+    total = spec.output_pixels_per_frame() * 4
+    frac = min(1.0, DUMP_LIMIT_BYTES / total)
+    rng = np.random.default_rng(0)
+    out = Path(dump_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for p, t in enumerate(planes):
+        ow, oh = spec.plane_dims(p)[2:4]
+        a = t[:, :ow]
+        if frac < 1.0:
+            rows = np.sort(rng.choice(oh, int(oh * frac), replace=False))
+            a = a[torch.from_numpy(rows).to(a.device)]
+        np.save(out / f"out_{'yuv'[p]}.npy", a.cpu().numpy().astype(np.float32))
+
+
+def measure_config(name, cfg, ctx, spec, K, warmup, dev, rank, world, barrier, want_e2e, e2e_steps, dump_dir=None):
     """Device-resident leg, roofline leg (the frame gather kernel alone: isolated launches and a back-to-back stream) and,
     optionally, the end-to-end leg of one config.  Returns a dict of raw measurements (this rank's; times are reduced
-    with MAX over ranks by the caller where the contract asks for it)."""
+    with MAX over ranks by the caller where the contract asks for it).  dump_dir: where the output frame of the last timed
+    step goes (dump_outputs)."""
     import torch
     import transform360_b200 as t360
     from transform360_b200 import synth
@@ -239,6 +262,8 @@ def measure_config(name, cfg, ctx, spec, K, warmup, dev, rank, world, barrier, w
     barrier()
     out = {"ms_total": e0.elapsed_time(e1), "launches": t360.kernel_launch_count() - launches0, "ring": ring,
            "plan_seconds": plan_seconds, "tiles": [list(ft.vft.plan_tile_counts(0)), list(ft.vft.plan_tile_counts(1))]}
+    if dump_dir is not None:  # before the legs below overwrite the output frames
+        dump_outputs(dump_dir, spec, fr.d_out[(K - 1) % 2])
 
     # ---- the dominant kernel alone: with the low-pass enabled a frame call also launches the blur kernels, so the gather
     # is timed through a second transform with the same geometry and the low-pass switched off (same jobs, same records)
@@ -367,7 +392,13 @@ def main():
     ap.add_argument("--skip-other-configs", action="store_true", help="do not add the short cfg3 / cfg4 legs (N=1 only)")
     ap.add_argument("--cpu-steps", type=int, default=12)
     ap.add_argument("--no-numa-bind", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output frame of the last timed step to DIR/out_{y,u,v}.npy "
+                    "(float32; a fixed sample of rows where the frame exceeds 64 MB), rank 0")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -420,7 +451,7 @@ def main():
     K = args.steps
     sampler = ClockSampler(local_rank) if rank == 0 else None
     m = measure_config(args.config, cfg, ctx, spec, K, args.warmup, dev, rank, world, barrier, not args.skip_e2e,
-                       args.e2e_steps or min(K, 100))
+                       args.e2e_steps or min(K, 100), args.dump_outputs if rank == 0 else None)
     (ms_total_max,) = max_over_ranks([m["ms_total"]])
     ms_per_step = ms_total_max / K
     value = in_px * K * world / (ms_total_max * 1e-3) / 1e6

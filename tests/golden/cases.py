@@ -4,6 +4,8 @@ Each case: context overrides on top of the reference filter defaults
 (vf_transform360.c:407-987), luma input dims, luma output dims.  yuv420p is assumed
 (chroma = ceil(dim / 2), vf_transform360.c:87-97), plan index 0 = luma, 1 = chroma.
 """
+import numpy as np
+
 L_CUBE32, L_CUBE23, L_FLAT, L_EQUIRECT, L_BARREL, L_BARREL_SPLIT, L_EAC = 0, 1, 2, 3, 4, 5, 6
 S_TB, S_LR, S_MONO = 0, 1, 2
 I_NEAREST, I_LINEAR, I_CUBIC, I_LANCZOS4 = 0, 1, 2, 4
@@ -77,6 +79,20 @@ SMALL = {
     "barrel_split_linear": dict(ov=dict(output_layout=L_BARREL_SPLIT, interpolation_alg=I_LINEAR,
                                         enable_low_pass_filter=0), inp=(512, 256), out=(180, 120)),
 }
+
+
+def plan_record(m, segments, centre_column=False):
+    """A plan as golden.json records it: hashes of the float map bit for bit, of the low-pass tile table (rectangle and
+    kernel lengths per tile) and of the taps.  segments: [(left, top, width, height, kx, ky)] in the reference's order.
+    centre_column also records the map without its centre column (side-by-side stereo outputs of odd width, DESIGN.md 7)."""
+    from oracle.ref_harness import sha16
+    bits = np.ascontiguousarray(m).view(np.uint32)
+    rects = np.array([(*s[:4], len(s[4]), len(s[5])) for s in segments], np.int32).reshape(-1, 6)
+    taps = np.concatenate([np.concatenate([s[4], s[5]]) for s in segments]) if segments else np.zeros(0, np.float32)
+    rec = {"shape": list(m.shape[:2]), "map": sha16(bits), "tiles": sha16(rects), "taps": sha16(taps.astype(np.float32))}
+    if centre_column:
+        rec["map_but_centre"] = sha16(np.delete(bits, m.shape[1] // 2, axis=1))
+    return rec
 
 
 def chroma(dim):

@@ -2,15 +2,21 @@
 against the libavfilter stand-in oracle/ffshim and driven by oracle/ff_driver.c, linked with
   * the reference library (oracle/_ref/libt360ref.so + cv2)            -> variant "ref"
   * the product          (transform360_b200/lib/libTransform360.so)    -> variant "b200".
-Same filter object code, same option strings; only libTransform360 differs.  Both .so files are prebuilt where
-/root/reference exists (make -C oracle ref) and travel to the GPU box."""
+Same filter object code, same option strings; only libTransform360 differs.  Both variants are built from the reference's
+filter source (make -C oracle ref), so the tests that use them skip where that source is absent.  The product's own
+CUDA-frame filter is checked against the sizes and frames the reference filter gave, recorded in tests/golden/golden.json."""
 import numpy as np
 import pytest
 
 from oracle import c_oracle as co
 from oracle import ff_harness as ff
+from oracle import ref_harness as rh
 
 needs_filters = pytest.mark.skipif(not (ff.available("ref") and ff.available("b200")), reason="oracle/_ref filter objects not built")
+
+
+def yuv_noise_frame(w, h):
+    return [co.noise_plane(w, h, 0, 3), co.noise_plane((w + 1) // 2, (h + 1) // 2, 1, 3), co.noise_plane((w + 1) // 2, (h + 1) // 2, 2, 3)]
 
 
 @needs_filters
@@ -50,7 +56,7 @@ def test_unmodified_reference_filter_gives_identical_frames_with_either_library(
     if not torch.cuda.is_available():
         pytest.fail("needs the B200 box")
     w, h = dims
-    planes = [co.noise_plane(w, h, 0, 3), co.noise_plane((w + 1) // 2, (h + 1) // 2, 1, 3), co.noise_plane((w + 1) // 2, (h + 1) // 2, 2, 3)]
+    planes = yuv_noise_frame(w, h)
     ref, b200 = ff.Filter("ref", args, w, h), ff.Filter("b200", args, w, h)
     assert (ref.out_w, ref.out_h) == (b200.out_w, b200.out_h)
     for frame in range(2):  # the first frame also runs generate_map (vf:346-352)
@@ -71,15 +77,19 @@ SIZE_CASES = [("cube_edge_length=70", (512, 256)), ("input_stereo_format=TB:cube
               ("input_stereo_format=lr:output_stereo_format=mono:output_layout=barrel:w=250:h=100", (1024, 128))]
 
 
+def size_key(args, dims):
+    return f"{args} {dims[0]}x{dims[1]}"
+
+
 @needs_cuda_filter
-def test_cuda_filter_option_table_and_output_size_without_a_device():
+def test_cuda_filter_option_table_and_output_size_without_a_device(golden):
     """transform360_cuda takes the reference filter's option strings (vf:407-987) and decides the same output size
-    (vf:167-304); graph configuration needs no GPU (the sampling plans wait for the first frame, like vf:346-352)."""
+    (vf:167-304) as the reference filter did (golden.json "reference_runs"); graph configuration needs no GPU (the
+    sampling plans wait for the first frame, like vf:346-352)."""
+    sizes = golden["reference_runs"]["filter_sizes"]
     for args, dims in SIZE_CASES:
         f = ff.CudaFilter(args, *dims, device=False)
-        if ff.available("ref"):
-            r = ff.Filter("ref", args, *dims)
-            assert (f.out_w, f.out_h) == (r.out_w, r.out_h), args
+        assert [f.out_w, f.out_h] == sizes[size_key(args, dims)], args
         f.close()
     assert (ff.CudaFilter("output_layout=eac_32:size=300x200", 512, 256, device=False).out_w) == 300  # honoured here (see the file header)
     for bad in ("interpolation_alg=bogus", "num_vertical_segments=1", "nonexistent=1", "yaw=400", "output_layout=eac_32:w=300",
@@ -107,10 +117,7 @@ def test_cuda_filter_defaults_are_the_reference_filters():
     assert expected <= names and names - expected == {"sync"}
 
 
-@needs_filters
-@needs_cuda_filter
-@pytest.mark.gpu
-@pytest.mark.parametrize("args,dims,extra", [
+CUDA_FRAME_CASES = [
     ("cube_edge_length=64:interpolation_alg=cubic:enable_low_pass_filter=0", (512, 256), ""),
     ("cube_edge_length=80:num_vertical_segments=15:num_horizontal_segments=8", (960, 480), ""),
     ("input_stereo_format=TB:output_layout=eac_32:w=192:h=128:interpolation_alg=lanczos4:num_vertical_segments=7", (512, 512), ":sync=0"),
@@ -118,19 +125,25 @@ def test_cuda_filter_defaults_are_the_reference_filters():
     ("cube_edge_length=48:width_scale_factor=2:height_scale_factor=2:enable_low_pass_filter=0", (512, 256), ":sync=0"),
     ("input_layout=cubemap_32:output_layout=equirect:w=512:h=256:enable_low_pass_filter=0", (384, 256), ""),
     ("output_layout=barrel:w=320:h=128:interpolation_alg=cubic", (640, 320), ""),
-])
-def test_cuda_frame_filter_matches_the_reference_filter(args, dims, extra):
-    """Device planes in, device planes out, whole frame per call on the device context's stream; the frames are those of
-    the reference's software filter (reference object code + cv2) for the same option string."""
+]
+
+
+@needs_cuda_filter
+@pytest.mark.gpu
+@pytest.mark.parametrize("args,dims,extra", CUDA_FRAME_CASES)
+def test_cuda_frame_filter_matches_the_reference_filter(args, dims, extra, golden):
+    """Device planes in, device planes out, whole frame per call on the device context's stream; the frames are those the
+    reference's software filter (reference object code + cv2) gave for the same option string (golden.json
+    "reference_runs", make_golden.py)."""
     import torch
     if not torch.cuda.is_available():
         pytest.fail("needs the B200 box")
     w, h = dims
-    planes = [co.noise_plane(w, h, 0, 3), co.noise_plane((w + 1) // 2, (h + 1) // 2, 1, 3), co.noise_plane((w + 1) // 2, (h + 1) // 2, 2, 3)]
-    ref = ff.Filter("ref", args, w, h)
+    planes = yuv_noise_frame(w, h)
+    want = golden["reference_runs"]["filter_frames"][args]
     stream = torch.cuda.Stream()
     gpu = ff.CudaFilter(args + extra, w, h, stream=stream)
-    assert (ref.out_w, ref.out_h) == (gpu.out_w, gpu.out_h)
+    assert [gpu.out_w, gpu.out_h] == want["size"]
     # decoder surfaces are pitched: 256-byte rows with the plane in the first columns
     dev = []
     for p in planes:
@@ -139,33 +152,30 @@ def test_cuda_frame_filter_matches_the_reference_filter(args, dims, extra):
         store[:, :p.shape[1]] = torch.from_numpy(p).cuda()
         dev.append(store[:, :p.shape[1]])
     torch.cuda.synchronize()
-    want = ref.filter(planes)
     for frame in range(3):
         got = gpu.filter(dev, out_pitch_pad=48)
         stream.synchronize()
         for p in range(3):
-            assert np.array_equal(got[p].cpu().numpy(), want[p]), f"plane {p} of frame {frame} differs ({args})"
-            assert bool((gpu.last_store[p][:, want[p].shape[1]:] == 0xA5).all()), "wrote beyond the plane's width"
-    ref.close()
+            assert list(got[p].shape) == want["shapes"][p]
+            assert rh.sha16(got[p].cpu().numpy()) == want["planes"][p], f"plane {p} of frame {frame} differs ({args})"
+            assert bool((gpu.last_store[p][:, got[p].shape[1]:] == 0xA5).all()), "wrote beyond the plane's width"
     gpu.close()
 
 
 @needs_cuda_filter
 @pytest.mark.gpu
-def test_cuda_frame_filter_gray8_and_refusals():
+def test_cuda_frame_filter_gray8_and_refusals(golden):
     import torch
     if not torch.cuda.is_available():
         pytest.fail("needs the B200 box")
-    from oracle import ref_harness as rh
     w, h = 512, 256
     y = co.noise_plane(w, h, 0, 5)
     gpu = ff.CudaFilter("cube_edge_length=64:interpolation_alg=cubic:enable_low_pass_filter=0", w, h, sw_format=ff.AV_PIX_FMT_GRAY8)
     got = gpu.filter([torch.from_numpy(y).cuda()])
     torch.cuda.synchronize()
-    if rh.REF_SO.exists():
-        t = rh.RefTransform(rh.default_context(interpolation_alg=2, enable_low_pass_filter=0))
-        assert t.generate_map(w, h, gpu.out_w, gpu.out_h, 0)
-        assert np.array_equal(got[0].cpu().numpy(), t.transform_plane(y, gpu.out_w, gpu.out_h, 0))
+    want = golden["reference_runs"]["gray8"]  # the reference's transform of the same plane at the same output size
+    assert [gpu.out_w, gpu.out_h] == want["size"]
+    assert rh.sha16(got[0].cpu().numpy()) == want["out_sha"]
     # a frame pool that has nothing to hand out: ENOMEM surfaces, nothing crashes
     rc = gpu.L.t360f_filter_cuda(gpu.h, (ff.C.c_void_p * 1)(got[0].data_ptr()), (ff.C.c_int * 1)(w), (ff.C.c_void_p * 1)(None), (ff.C.c_int * 1)(0))
     assert rc == -12

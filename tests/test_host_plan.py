@@ -12,7 +12,7 @@ import pytest
 import transform360_b200 as t360
 from oracle import c_oracle as co
 from oracle import ref_harness as rh
-from tests.golden.cases import FULL, SMALL, plane_dims
+from tests.golden.cases import FULL, SMALL, plan_record, plane_dims
 from transform360_b200 import build as t360_build
 
 ROOT = Path(__file__).resolve().parents[1]
@@ -43,7 +43,7 @@ def test_library_exports_declared_abi():
         assert getattr(lib, s)
 
 
-def test_context_layout_matches_reference_header():
+def test_context_layout_matches_reference_header(tmp_path):
     assert ctypes.sizeof(t360.FrameTransformContext) == 112
     assert t360.FrameTransformContext.interpolation_alg.offset == 28
     assert t360.FrameTransformContext.kernel_adjust_factor.offset == 108
@@ -57,7 +57,7 @@ def test_context_layout_matches_reference_header():
     prog = '#include "Transform360/VideoFrameTransformHandler.h"\n#include <stddef.h>\n#include <stdio.h>\n' \
            'int main(void){printf("%zu %zu %zu", sizeof(FrameTransformContext), offsetof(FrameTransformContext, interpolation_alg),' \
            ' offsetof(FrameTransformContext, kernel_adjust_factor));return 0;}'
-    exe = Path("/tmp/t360_abi_probe")
+    exe = tmp_path / "t360_abi_probe"
     subprocess.run(["gcc", "-std=c11", "-x", "c", "-", "-I", str(ROOT / "include"), "-o", str(exe)], input=prog, text=True, check=True)
     assert subprocess.run([str(exe)], capture_output=True, text=True).stdout == "112 28 108"
 
@@ -138,23 +138,15 @@ def test_full_size_plan_matches_golden(name, golden):
     hp.close()
 
 
-@pytest.mark.skipif(not rh.ref_available(), reason="oracle/_ref not built")
-def test_plan_matches_live_reference_with_odd_parameters():
-    ov = dict(fixed_yaw=123.4, fixed_pitch=-67.8, fixed_roll=179.0, fixed_cube_offcenter_x=0.2, fixed_cube_offcenter_y=-0.15,
-              fixed_cube_offcenter_z=-0.4, num_vertical_segments=12, num_horizontal_segments=7, expand_coef=1.05,
-              kernel_height_scale_factor=1.7, kernel_adjust_factor=1.3, output_layout=t360.LAYOUT_EAC_32)
-    ctx, rctx = t360.make_context(**ov), rh.default_context(**ov)
-    ref = rh.RefTransform(rctx)
-    assert ref.generate_map(700, 350, 300, 200, 0)
-    hp = t360.HostPlan(ctx, 700, 350, 300, 200)
-    assert np.array_equal(hp.map.view(np.uint32), ref.map(0).view(np.uint32))
-    a, b = hp.segments(), ref.segments(0)
-    assert len(a) == len(b)
-    for s, r in zip(a, b):
-        assert s[:4] == r[:4]
-        assert np.array_equal(s[4].view(np.uint32), r[4].view(np.uint32))
-        assert np.array_equal(s[5].view(np.uint32), r[5].view(np.uint32))
-    ref.close()
+ODD_PARAMETERS = dict(fixed_yaw=123.4, fixed_pitch=-67.8, fixed_roll=179.0, fixed_cube_offcenter_x=0.2, fixed_cube_offcenter_y=-0.15,
+                      fixed_cube_offcenter_z=-0.4, num_vertical_segments=12, num_horizontal_segments=7, expand_coef=1.05,
+                      kernel_height_scale_factor=1.7, kernel_adjust_factor=1.3, output_layout=t360.LAYOUT_EAC_32)
+
+
+def test_plan_matches_live_reference_with_odd_parameters(golden):
+    """Map, tile table and taps of a 700x350 -> 300x200 plan against the reference's own (golden.json "reference_runs")."""
+    hp = t360.HostPlan(t360.make_context(**ODD_PARAMETERS), 700, 350, 300, 200)
+    assert plan_record(hp.map, hp.segments()) == golden["reference_runs"]["odd_parameters"]
     hp.close()
 
 
@@ -192,65 +184,63 @@ def _random_context(rng):
     return ov
 
 
-@pytest.mark.skipif(not rh.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("seed", [1, 2, 3])
-def test_random_parameter_sweep_against_the_compiled_reference(seed):
-    """Random contexts over the whole option space (layouts both ways, stereo, rotation, off-centre, scale factors,
-    low-pass parameters, odd sizes): the planner's float map, tile table and taps must equal, bit for bit, what the
-    reference's own object code (oracle/_ref) produces -- and fail where it fails.  One documented exception: the
-    centre column of a side-by-side stereo output of odd render width, where the reference reads an uninitialised face
-    basis (DESIGN.md 7); there the planner must equal the C oracle instead.  (1200 cases of this sweep found the
-    out-of-range face index and the negative-sigma refusal fixed alongside this test.)"""
+def _plan_sweep_cases(seed):
+    """(overrides, (in_w, in_h, out_w, out_h)) of the random parameter sweep."""
     rng = np.random.default_rng(seed)
-    compared = 0
     for _ in range(50):
         ov = _random_context(rng)
         iw, ih = int(rng.integers(64, 400)) * 2, int(rng.integers(32, 200)) * 2
         ow, oh = int(rng.integers(24, 160)) * 2, int(rng.integers(16, 120)) * 2
-        ctx, rctx = t360.make_context(**ov), rh.default_context(**ov)
-        ref = rh.RefTransform(rctx)
-        ok_ref = bool(ref.generate_map(iw, ih, ow, oh, 0))
+        yield ov, (iw, ih, ow, oh)
+
+
+@pytest.mark.parametrize("seed", [1, 2, 3])
+def test_random_parameter_sweep_against_the_compiled_reference(seed, golden):
+    """Random contexts over the whole option space (layouts both ways, stereo, rotation, off-centre, scale factors,
+    low-pass parameters, odd sizes): the planner's float map, tile table and taps must equal, bit for bit, what the
+    reference's own object code produced (golden.json "reference_runs", make_golden.py) -- and fail where it failed.  One
+    documented exception: the centre column of a side-by-side stereo output of odd render width, where the reference reads
+    an uninitialised face basis (DESIGN.md 7); there the planner must equal the C oracle instead.  (1200 cases of this
+    sweep found the out-of-range face index and the negative-sigma refusal fixed alongside this test.)"""
+    cases = list(_plan_sweep_cases(seed))
+    runs = golden["reference_runs"]["plan_sweep"][str(seed)]
+    assert len(runs) == len(cases)
+    compared = 0
+    for (ov, dims), want in zip(cases, runs):
         try:
-            hp = t360.HostPlan(ctx, iw, ih, ow, oh)
+            hp = t360.HostPlan(t360.make_context(**ov), *dims)
         except ValueError:
             hp = None
-        assert ok_ref == (hp is not None), f"status differs for {ov} {(iw, ih, ow, oh)}"
+        assert (want is not None) == (hp is not None), f"status differs for {ov} {dims}"
         if hp is None:
-            ref.close()
             continue
-        got, want = hp.map.view(np.uint32), ref.map(0).view(np.uint32)
-        assert got.shape == want.shape
-        differ = got != want
-        if differ.any():
-            mw = got.shape[1]
+        got = plan_record(hp.map, hp.segments(), centre_column=True)
+        if got["map"] != want["map"]:
+            mw = got["shape"][1]
             lr_centre = ov["input_stereo_format"] != 2 and ov["output_stereo_format"] == 1 and mw % 2 == 1
-            assert lr_centre and not np.delete(differ, mw // 2, axis=1).any(), f"map differs for {ov} {(iw, ih, ow, oh)}"
-            assert np.array_equal(got, co.generate_map(rctx, iw, ih, ow, oh).view(np.uint32)), "planner != C oracle on the centre column"
-        a, b = hp.segments(), ref.segments(0)
-        assert len(a) == len(b)
-        for s, r in zip(a, b):
-            assert s[:4] == r[:4]
-            assert np.array_equal(s[4].view(np.uint32), r[4].view(np.uint32)) and np.array_equal(s[5].view(np.uint32), r[5].view(np.uint32))
+            assert lr_centre and got["map_but_centre"] == want["map_but_centre"], f"map differs for {ov} {dims}"
+            oracle_map = co.generate_map(rh.default_context(**ov), *dims)
+            assert np.array_equal(hp.map.view(np.uint32), oracle_map.view(np.uint32)), "planner != C oracle on the centre column"
+            got["map"] = want["map"]
+        assert got == want, f"plan differs for {ov} {dims}"
         compared += 1
-        ref.close()
         hp.close()
     assert compared >= 40
 
 
-@pytest.mark.skipif(not rh.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("nh,adjust", [(0, 1), (-2, 1), (0, 0), (-3, 0)])
-def test_non_positive_horizontal_segment_counts_follow_the_reference(nh, adjust):
+NON_POSITIVE_HORIZONTAL_SEGMENTS = [(0, 1), (-2, 1), (0, 0), (-3, 0)]
+
+
+def _non_positive_overrides(nh, adjust):
+    return dict(interpolation_alg=2, enable_low_pass_filter=1, num_vertical_segments=5, num_horizontal_segments=nh, adjust_kernel=adjust)
+
+
+@pytest.mark.parametrize("nh,adjust", NON_POSITIVE_HORIZONTAL_SEGMENTS)
+def test_non_positive_horizontal_segment_counts_follow_the_reference(nh, adjust, golden):
     """Not an error in the reference: with adjust_kernel its tile loop does not run (no tiles: the low-pass output stays
-    zero), without adjust_kernel the value is ignored (cpp:224-235)."""
-    ov = dict(interpolation_alg=2, enable_low_pass_filter=1, num_vertical_segments=5, num_horizontal_segments=nh, adjust_kernel=adjust)
-    ctx, rctx = t360.make_context(**ov), rh.default_context(**ov)
-    ref = rh.RefTransform(rctx)
-    assert ref.generate_map(320, 160, 96, 64, 0)
-    hp = t360.HostPlan(ctx, 320, 160, 96, 64)
-    a, b = hp.segments(), ref.segments(0)
-    assert len(a) == len(b) == (0 if adjust else 5)
-    for s, r in zip(a, b):
-        assert s[:4] == r[:4] and np.array_equal(s[4].view(np.uint32), r[4].view(np.uint32)) and np.array_equal(s[5].view(np.uint32), r[5].view(np.uint32))
-    assert np.array_equal(hp.map.view(np.uint32), ref.map(0).view(np.uint32))
-    ref.close()
+    zero), without adjust_kernel the value is ignored (cpp:224-235).  Against the reference's plan (golden.json)."""
+    hp = t360.HostPlan(t360.make_context(**_non_positive_overrides(nh, adjust)), 320, 160, 96, 64)
+    segs = hp.segments()
+    assert len(segs) == (0 if adjust else 5)
+    assert plan_record(hp.map, segs) == golden["reference_runs"]["non_positive_horizontal_segments"][f"{nh},{adjust}"]
     hp.close()

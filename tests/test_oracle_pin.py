@@ -4,14 +4,15 @@ The reference has no tests or golden vectors of its own (SURVEY.md 4), so the pi
 (a) tests/golden/golden.json -- outputs of THE REFERENCE ITSELF run in the build container
     (oracle/_ref = unmodified reference sources + oracle/shim, driving cv2 4.13.0; generator
     tests/golden/make_golden.py) -- checked without needing /root/reference at run time;
-(b) live comparison with oracle/_ref and cv2 where those are present.
+(b) further runs of the reference recorded in the same file ("reference_runs": other seeds, planes and contexts),
+    and live comparison with cv2.
 """
 import numpy as np
 import pytest
 
 from oracle import c_oracle as co
 from oracle import ref_harness as rh
-from tests.golden.cases import FULL, SMALL, plane_dims
+from tests.golden.cases import FULL, SMALL, plan_record, plane_dims
 
 cv2 = pytest.importorskip("cv2")
 
@@ -175,25 +176,30 @@ def test_area_resize_enlarging_vs_cv2():
         assert np.array_equal(co.resize_area(src, dw, dh), cv2.resize(src, (dw, dh), interpolation=cv2.INTER_AREA)), (sw, sh, dw, dh)
 
 
-@pytest.mark.skipif(not rh.ref_available(), reason="oracle/_ref not built")
-def test_scale_factors_below_one_end_to_end_vs_live_reference():
-    """width/height_scale_factor < 1: render at the smaller map size, then INTER_AREA *up* (ref:755-777)."""
-    for ov, dims in ((dict(width_scale_factor=0.5, height_scale_factor=0.5, interpolation_alg=2), (320, 160, 96, 64)),
-                     (dict(width_scale_factor=0.75, height_scale_factor=1.0, interpolation_alg=1, enable_low_pass_filter=0), (256, 128, 96, 64)),
-                     (dict(width_scale_factor=2.0, height_scale_factor=0.6, interpolation_alg=4, output_layout=rh.LAYOUT_EAC_32), (300, 150, 60, 50)),
-                     (dict(width_scale_factor=0.9, height_scale_factor=0.8, interpolation_alg=0, output_layout=rh.LAYOUT_BARREL), (256, 128, 100, 40))):
+# width/height_scale_factor < 1 end to end: (context overrides, (in_w, in_h, out_w, out_h))
+SCALE_BELOW_ONE = ((dict(width_scale_factor=0.5, height_scale_factor=0.5, interpolation_alg=2), (320, 160, 96, 64)),
+                   (dict(width_scale_factor=0.75, height_scale_factor=1.0, interpolation_alg=1, enable_low_pass_filter=0), (256, 128, 96, 64)),
+                   (dict(width_scale_factor=2.0, height_scale_factor=0.6, interpolation_alg=4, output_layout=rh.LAYOUT_EAC_32), (300, 150, 60, 50)),
+                   (dict(width_scale_factor=0.9, height_scale_factor=0.8, interpolation_alg=0, output_layout=rh.LAYOUT_BARREL), (256, 128, 100, 40)))
+
+
+def _prefill(ctx):
+    return 9 if ctx.output_layout in (rh.LAYOUT_BARREL, rh.LAYOUT_BARREL_SPLIT) else 0
+
+
+def test_scale_factors_below_one_end_to_end_vs_live_reference(golden):
+    """width/height_scale_factor < 1: render at the smaller map size, then INTER_AREA *up* (ref:755-777); against the
+    reference's own outputs for the same planes (golden.json "reference_runs", make_golden.py)."""
+    runs = golden["reference_runs"]["scale_below_one"]
+    assert len(runs) == len(SCALE_BELOW_ONE)
+    for (ov, dims), want in zip(SCALE_BELOW_ONE, runs):
         ctx = rh.default_context(**ov)
         iw, ih, ow, oh = dims
-        ref = rh.RefTransform(ctx)
         for idx in (0, 1):
-            assert ref.generate_map(iw, ih, ow, oh, idx)
             plan = co.OraclePlan(ctx, iw, ih, ow, oh)
             src = co.noise_plane(iw, ih, plane=idx, frame=5)
-            pre = 9 if ctx.output_layout in (rh.LAYOUT_BARREL, rh.LAYOUT_BARREL_SPLIT) else 0
-            want = ref.transform_plane(src, ow, oh, idx, image_plane=idx, prefill=pre)
-            got = co.transform_plane(ctx, plan, src, ow, oh, map_index=idx, prefill=pre)
-            assert np.array_equal(got, want), (ov, idx)
-        ref.close()
+            got = co.transform_plane(ctx, plan, src, ow, oh, map_index=idx, prefill=_prefill(ctx))
+            assert rh.sha16(got) == want[idx], (ov, idx)
 
 
 def test_itab_sums():
@@ -222,67 +228,61 @@ def test_sepfilter_arithmetic_vs_cv2(sx, sy):
     assert np.array_equal(tile[100:228, 300:540], want[100:228, 300:540])
 
 
-@pytest.mark.skipif(not rh.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("name", ["lp_tiles", "eac_tb_lanczos", "offcenter_adjust", "cube_to_equirect", "barrel"])
-def test_oracle_vs_live_reference(name):
-    """Same comparison as the golden test but against the compiled reference run live (different frame seed)."""
+LIVE_CASES = ["lp_tiles", "eac_tb_lanczos", "offcenter_adjust", "cube_to_equirect", "barrel"]
+
+
+@pytest.mark.parametrize("name", LIVE_CASES)
+def test_oracle_vs_live_reference(name, golden):
+    """Same comparison as the golden test but with another frame seed and planes 0 and 2, down to the tile table and the
+    taps, against the reference's own run of them (golden.json "reference_runs", make_golden.py)."""
     case = SMALL[name]
     ctx = _ctx(case)
-    ref = rh.RefTransform(ctx)
+    runs = golden["reference_runs"]["live_cases"][name]
     for plane in (0, 2):
         iw, ih, ow, oh, idx = plane_dims(case, plane)
-        assert ref.generate_map(iw, ih, ow, oh, idx)
         plan = co.OraclePlan(ctx, iw, ih, ow, oh)
-        assert np.array_equal(plan.map.view(np.uint32), ref.map(idx).view(np.uint32))
-        rs = ref.segments(idx)
         mine = co.plan_as_list(plan.segs, plan.nsegs, plan.taps) if plan.nsegs else []
-        assert len(rs) == len(mine)
-        for a, b in zip(rs, mine):
-            assert a[:4] == b[:4]
-            assert np.array_equal(a[4].view(np.uint32), b[4].view(np.uint32))
-            assert np.array_equal(a[5].view(np.uint32), b[5].view(np.uint32))
+        assert plan_record(plan.map, mine) == runs[str(plane)]["plan"], f"plane {plane}: plan differs from the reference"
         src = co.noise_plane(iw, ih, plane=plane, frame=17)
-        barrel = ctx.output_layout in (rh.LAYOUT_BARREL, rh.LAYOUT_BARREL_SPLIT)
-        want = ref.transform_plane(src, ow, oh, idx, image_plane=plane, prefill=9 if barrel else 0)
-        got = co.transform_plane(ctx, plan, src, ow, oh, map_index=idx, prefill=9 if barrel else 0)
-        assert np.array_equal(got, want)
-    ref.close()
+        got = co.transform_plane(ctx, plan, src, ow, oh, map_index=idx, prefill=_prefill(ctx))
+        assert rh.sha16(got) == runs[str(plane)]["out_sha"], f"plane {plane}: pixels differ from the reference"
 
 
-@pytest.mark.skipif(not rh.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("seed", [11, 12])
-def test_random_end_to_end_sweep_against_the_live_reference(seed):
-    """Random contexts over the whole option space, end to end: the C restatement must produce the bytes the reference's
-    own object code + cv2 produce.  (1300 cases of this sweep, offline, found the NaN-coordinate rule pinned above; the
-    only remaining difference is the centre column of side-by-side stereo outputs of odd render width, where the
-    reference reads an uninitialised face basis -- those contexts are skipped here, DESIGN.md 7.)"""
+def _e2e_sweep_cases(seed):
+    """(overrides, (in_w, in_h, out_w, out_h), plan index) of the end-to-end sweep.  Side-by-side stereo outputs of odd
+    render width are left out: there the reference reads an uninitialised face basis (DESIGN.md 7)."""
     from tests.test_host_plan import _random_context
     rng = np.random.default_rng(1000 + seed)
-    compared = 0
     for _ in range(25):
         ov = _random_context(rng)
         iw, ih = int(rng.integers(64, 300)) * 2, int(rng.integers(32, 150)) * 2
         ow, oh = int(rng.integers(24, 120)) * 2 + int(rng.random() < 0.25), int(rng.integers(16, 90)) * 2 + int(rng.random() < 0.25)
         idx = int(rng.integers(0, 2))
-        ctx = rh.default_context(**ov)
-        sw, _ = co.scaled_dims(ctx, ow, oh)
+        sw, _ = co.scaled_dims(rh.default_context(**ov), ow, oh)
         if ov["input_stereo_format"] != rh.STEREO_FORMAT_MONO and ov["output_stereo_format"] == rh.STEREO_FORMAT_LR and sw % 2 == 1:
             continue
-        ref = rh.RefTransform(ctx)
-        if not ref.generate_map(iw, ih, ow, oh, idx):
-            ref.close()
+        yield ov, (iw, ih, ow, oh), idx
+
+
+@pytest.mark.parametrize("seed", [11, 12])
+def test_random_end_to_end_sweep_against_the_live_reference(seed, golden):
+    """Random contexts over the whole option space, end to end: the C restatement must produce the bytes the reference's
+    own object code + cv2 produced for them (golden.json "reference_runs", make_golden.py).  (1300 cases of this sweep,
+    offline, found the NaN-coordinate rule pinned above.)"""
+    cases = list(_e2e_sweep_cases(seed))
+    runs = golden["reference_runs"]["e2e_sweep"][str(seed)]
+    assert len(runs) == len(cases)
+    compared = 0
+    for (ov, (iw, ih, ow, oh), idx), want in zip(cases, runs):
+        if want is None:  # the reference refused the plan or the frame
             continue
+        ctx = rh.default_context(**ov)
         plan = co.OraclePlan(ctx, iw, ih, ow, oh)
         src = co.noise_plane(iw, ih, plane=idx, frame=seed)
-        pre = 9 if ctx.output_layout in (rh.LAYOUT_BARREL, rh.LAYOUT_BARREL_SPLIT) else 0
         try:
-            want = ref.transform_plane(src, ow, oh, idx, image_plane=idx, prefill=pre)
-            got = co.transform_plane(ctx, plan, src, ow, oh, map_index=idx, prefill=pre)
+            got = co.transform_plane(ctx, plan, src, ow, oh, map_index=idx, prefill=_prefill(ctx))
         except RuntimeError:  # scale factors < 1 are not restated (INTER_AREA enlarging)
-            ref.close()
             continue
-        assert np.array_equal(got, want), f"{(got != want).sum()} px differ for {ov} {(iw, ih, ow, oh)} plan {idx}"
+        assert rh.sha16(got) == want, f"pixels differ for {ov} {(iw, ih, ow, oh)} plan {idx}"
         compared += 1
-        ref.close()
     assert compared >= 15
-
